@@ -14,6 +14,10 @@ per step).
 Prints ONE JSON line (rank 0).  `value` = nominal ray-samples/s with the frame's uniforms
 resident in HBM; `e2e` = the same through NeRFRender.render_image with HOST buffers (uniforms
 copied from pinned memory, image copied back) inside the timed region.
+
+`--dump-outputs DIR` writes what the last timed step returned (render: colour and depth of every frame of the step;
+train: the loss, the render outputs and the updated weights) as DIR/<name>.npy.  Weights, cameras, uniforms and
+batches are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,6 +49,35 @@ NET_CFG = dict(_target_="neddf.network.NeDDF", embed_pos_rank=10, embed_dir_rank
 RENDER_CFG = dict(sample_coarse=S_COARSE, sample_fine=S_FINE, dist_near=2.0, dist_far=6.0, max_dist=6.0,
                   use_coarse_network=False, sampling_type="cone")
 WEIGHT_SEED = 3408
+DUMP_LIMIT = 64 << 20  # bytes of --dump-outputs in all
+
+
+def write_outputs(path: str, arrays) -> None:
+    """--dump-outputs: every array as <path>/<name>.npy, float64 kept, everything else as float32."""
+    import numpy as np
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT})")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
+def frame_outputs(outs, n_pix: int):
+    """Colour [frames, pixels, 3] and depth [frames, pixels, 1] of one step's frames on the host (each frame either
+    render_pixels' dict or the all-gathered [pixels, 4] colour + depth tiles).  When the frames do not fit half of
+    DUMP_LIMIT, every frame keeps the same fixed, seeded sample of pixels, listed in ``pixel_index``."""
+    import numpy as np
+    img = torch.stack([o if torch.is_tensor(o) else torch.cat([o["color"], o["depth"]], 1) for o in outs]).cpu().numpy()
+    res = {}
+    keep = (DUMP_LIMIT // 2) // (img.shape[0] * img.shape[2] * img.itemsize)
+    if keep < n_pix:
+        idx = np.sort(np.random.default_rng(0).choice(n_pix, keep, replace=False))
+        img = img[:, idx]
+        res["pixel_index"] = idx.astype(np.float64)
+    res["color"], res["depth"] = img[..., :3], img[..., 3:]
+    return res
 
 
 def synthetic_pose(seed: int):
@@ -358,6 +391,7 @@ def run_train(args):
         raise SystemExit("bench.py: no CUDA device - the training path has no CPU implementation")
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(0)
+    torch.manual_seed(0)  # render_rays draws the training uniforms from torch's generator: same run, same numbers
     sd, _ = seeded_state_dict()
     render = neddf_b200.NeRFRender(network_config=NET_CFG, **RENDER_CFG)
     render.load_state_dict(sd)
@@ -383,37 +417,42 @@ def run_train(args):
         opt.zero_grad(set_to_none=True)
         loss.backward()
         opt.step()
-        return loss
+        return loss, out
 
     def step_device(i):
         return one_step(*resident[i % n_batches])
 
     def step_e2e(i):
         uv, color, mask = (x.to(dev, non_blocking=True) for x in host[i % n_batches])
-        return float(one_step(uv, color, mask).item())  # the loss the trainer logs (nerf_trainer.py:124)
+        return float(one_step(uv, color, mask)[0].item())  # the loss the trainer logs (nerf_trainer.py:124)
 
     def timed(fn, steps):
+        """(ms per step, what the last step returned)"""
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            fn(i)
+            last = fn(i)
         e1.record()
         torch.cuda.synchronize()
-        return e0.elapsed_time(e1) / steps
+        return e0.elapsed_time(e1) / steps, last
 
     for i in range(args.warmup):
         step_device(i)
     sampler = ClockSampler(0)
     sampler.start()
     launches0 = L.lib().neddf_launch_count()
-    ms_step = timed(step_device, args.steps)
+    ms_step, (loss, out) = timed(step_device, args.steps)
     launches = L.lib().neddf_launch_count() - launches0
     clocks = sampler.stop()
     render.check_status()
+    if args.dump_outputs:  # the loss, the render outputs and the weights after the optimiser step
+        dump = {"loss": loss.detach().cpu().numpy()}
+        dump.update({k: v.detach().cpu().numpy() for k, v in out.items()})
+        dump.update({"param." + k: v.detach().cpu().numpy() for k, v in render.network_fine.state_dict().items()})
     for i in range(2):
         step_e2e(i)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     value = TRAIN_RAYS * NOMINAL_PER_RAY / (ms_step * 1e-3)
     evals = TRAIN_RAYS * EVALS_PER_RAY
     peaks = {}
@@ -430,6 +469,8 @@ def run_train(args):
         cpu = {"value": v, "unit": "ray-samples/s", "cores": threads, "kind": "port",
                "sample": f"16 rays: forward + autograd backward + Adam ({dt:.1f} s)"}
     engine = render.network_fine.resolved_engine(dev)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps({
         "metric": metric, "value": value, "unit": "ray-samples/s", "n_gpus": 1, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -464,7 +505,14 @@ def main():
                     help="early ray termination threshold on the transmittance (BASELINE.json configs[4]; 0 = off = "
                          "the reference's behaviour, the default workload)")
     ap.add_argument("--segments", type=int, default=4, help="depth segments of the fine pass when --eps > 0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB; seeded inputs, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; --impl reference has none")
     if args.warmup < 3:
         args.warmup = 3  # timing rules: W >= 3
     if args.workload == "train":
@@ -556,7 +604,7 @@ def main():
             render.network_fine._profile_events = []
         ev0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -567,7 +615,7 @@ def main():
         if profile:
             evs = render.network_fine._profile_events
             render.network_fine._profile_events = None
-        return float(t.item()), evs
+        return float(t.item()), evs, last
 
     for _ in range(args.warmup):
         step_device()
@@ -576,9 +624,12 @@ def main():
         sampler.start()
     render.termination_stats()  # reset the executed / nominal counters after the warm-up
     launches0 = L.lib().neddf_launch_count()
-    ms_total, evs = timed(step_device, args.steps, profile=True)
+    ms_total, evs, last = timed(step_device, args.steps, profile=True)
     launches = L.lib().neddf_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    # copied now: the renders below may reuse the buffers behind the last step's outputs
+    dump = frame_outputs(last, n_pix) if args.dump_outputs and rank == 0 else None
+    del last
     render.check_status()
     term = render.termination_stats()  # fine-pass evaluations of this rank inside the timed region
     if world > 1:
@@ -626,7 +677,7 @@ def main():
     # end to end through the public API with host buffers
     for _ in range(2):
         step_e2e()
-    ms_e2e, _ = timed(step_e2e, max(1, args.steps))
+    ms_e2e, _, _ = timed(step_e2e, max(1, args.steps))
     ms_e2e /= max(1, args.steps)
     e2e_value = rays_per_step * NOMINAL_PER_RAY / (ms_e2e * 1e-3)
     h2d = n_frames * count * (S_COARSE + 1 + S_FINE + 1) * 4 + n_frames * 16 * 4
@@ -642,7 +693,7 @@ def main():
             return gather_tiles(torch.cat([flat["color"], flat["depth"]], 1), n_pix)
 
         one_frame()
-        ms_frame, _ = timed(one_frame, max(3, args.steps))
+        ms_frame, _, _ = timed(one_frame, max(3, args.steps))
         ms_frame /= max(3, args.steps)
         strong = {"frame_ms": ms_frame, "ray_samples_per_s": n_pix * NOMINAL_PER_RAY / (ms_frame * 1e-3),
                   "note": "one 800x800 frame sharded over the ranks + the all-gather of the image tiles"}
@@ -659,6 +710,8 @@ def main():
 
     if rank == 0:
         engine = render.network_fine.resolved_engine(dev)
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         line = {
             "metric": "ray-samples/s (800x800x192)", "value": value, "unit": "ray-samples/s", "n_gpus": n_gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_step, "higher_is_better": True,

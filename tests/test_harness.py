@@ -1,15 +1,16 @@
 """The reference's own evaluation entry point, unmodified, against the B200 classes - as far as a box without a GPU
 can take it (VERDICT round 1, item 7).
 
-`python -m neddf_b200.launch neddf/scripts/run_eval.py <run dir>` is executed in a subprocess from /root/reference
+`python -m neddf_b200.launch neddf/scripts/run_eval.py <run dir>` is executed in a subprocess from oracle/_ref/neddf,
+the copy of the reference's scripts, configs, dataset and checkpoint that build() stages (oracle/reference_tree.py),
 with Hydra / omegaconf / scikit-image stand-ins (tests/harness_stub: DictConfig and ListConfig are NOT dict / list
 subclasses, `instantiate` honours `_recursive_=False`, like the real packages that are not installable here).  The
 script composes the saved `.hydra/config.yaml`, Hydra instantiates the reference's NeRFTrainer, which instantiates
 `neddf.render.NeRFRender` with the un-instantiated network node (nerf_trainer.py:32-36) - rebound to neddf_b200 by
 the launcher -, builds Adam over get_parameters_list(), loads the real checkpoint (base_trainer.py:121, strict) and
 calls render_all -> render_image.  That last call is the kernel boundary: on this GPU-less box it must fail loudly
-from neddf_b200 (no CPU fallback).  /root/reference does not exist on the GPU box, so the GPU half of this harness
-cannot run there; the image path itself is parity-tested on the GPU against the reference's image golden."""
+from neddf_b200 (no CPU fallback).  On a GPU machine the runs would render and train for real, so these tests are
+CPU-only; the image path itself is parity-tested on the GPU against the reference's image golden."""
 import os
 import shutil
 import subprocess
@@ -18,12 +19,13 @@ import sys
 import pytest
 import torch
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
+REF = os.path.join(REPO, "oracle", "_ref", "neddf")
+NEEDS_REF = "needs oracle/_ref/neddf, which build() stages from a ueda0319/neddf checkout"
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pretrained", "bunny_smoke")), reason="needs /root/reference")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pretrained", "bunny_smoke")), reason=NEEDS_REF)
 def test_run_eval_reaches_the_kernel_boundary(tmp_path):
     if torch.cuda.is_available():
         pytest.skip("CPU harness: on a GPU box the run would render 50 full frames")
@@ -45,7 +47,7 @@ def test_run_eval_reaches_the_kernel_boundary(tmp_path):
     assert (run_dir / "eval").is_dir()  # run_eval.py:41-42 created its output directory before rendering
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "data", "bunny_smoke")), reason="needs /root/reference")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "data", "bunny_smoke")), reason=NEEDS_REF)
 @pytest.mark.parametrize("argv,patch", [
     ([], "0"),                                                                                    # config/config.yaml defaults: NeDDF
     (["network=nerf", "render=nerf_render", "loss=nerf_loss", "trainer=nerf_trainer"], "1"),  # NeRF groups + trainer glue

@@ -1,6 +1,5 @@
 """CPU: host-side mirror of the reference interface (no kernels run)."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -8,7 +7,7 @@ import torch
 
 import neddf_b200
 from oracle import neddf_oracle as orc
-from tests.helpers import Case
+from tests.helpers import GOLDEN, Case
 
 
 def test_state_dict_surface_matches_reference_checkpoint():
@@ -58,11 +57,12 @@ def test_neus_module_surface_matches_the_reference():
     """Same constructor, parameter names / shapes and initial values as neddf.network.NeuS for the same torch seed;
     NeRFRender resolves the reference's _target_ to it; the C ABI reports the same layer shapes and refusals."""
     import ctypes as C
+    import json
 
     from neddf_b200 import _lib as L
     from oracle import neddf_oracle as orc
-    kw = dict(embed_pos_rank=5, embed_dir_rank=3, sdf_layer_count=6, col_layer_count=3, activation_type="tanhExp",
-              init_variance=0.45, skips=[1, 3])
+    from tests.golden.make_host_golden import NEUS_KW as kw
+    from tests.golden.make_host_golden import tensor_digest, tensor_sample
     torch.manual_seed(7)
     net = neddf_b200.NeuS(**kw)
     sd = net.state_dict()
@@ -71,17 +71,12 @@ def test_neus_module_surface_matches_the_reference():
     for n, cin, cout in shapes:  # torch nn.Linear keeps [out, in]
         assert tuple(sd[n + ".weight"].shape) == (cout, cin) and tuple(sd[n + ".bias"].shape) == (cout,)
     assert abs(float(sd["variance"]) - 0.45) < 1e-7
-    ref_root = "/root/reference"
-    if os.path.isdir(ref_root):
-        sys.path.insert(0, ref_root)
-        try:
-            from neddf.network import NeuS as RefNeuS
-            torch.manual_seed(7)
-            ref = RefNeuS(**kw).state_dict()
-        finally:
-            sys.path.remove(ref_root)
-        assert list(ref) == list(sd)
-        assert all(torch.equal(ref[k], sd[k]) for k in ref)
+    # the reference's NeuS(**kw) after the same seed (tests/golden/make_host_golden.py): key order, values bit for bit
+    z = np.load(os.path.join(GOLDEN, "case_host.npz"))
+    assert json.loads(str(z["neus_keys"])) == list(sd)
+    for i, (k, v) in enumerate(sd.items()):
+        assert np.array_equal(tensor_sample(v), z[f"neus_sample_{i}"]), k
+    assert [tensor_digest(v) for v in sd.values()] == json.loads(str(z["neus_sha256"]))
     r = neddf_b200.NeRFRender(network_config={"_target_": "neddf.network.NeuS", **kw}, use_coarse_network=False)
     assert isinstance(r.network_fine, neddf_b200.NeuS) and r.network_coarse is r.network_fine
     assert len(r.get_parameters_list()) == 2 * len(shapes) + 1
@@ -111,23 +106,29 @@ def test_camera_standin_matches_reference_pose():
     assert np.allclose(cam2.T.numpy(), [1, 2, 3])
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir("/root/reference/neddf"), reason="reference tree not present")
 def test_install_rebinds_reference_targets(repo_root):
     """neddf_b200.install makes the saved `_target_` strings resolve to the B200 classes and the
-    pretrained checkpoint loads unchanged (subprocess: do not pollute this interpreter's modules)."""
+    pretrained checkpoint loads unchanged (subprocess: do not pollute this interpreter's modules).
+    The reference's packages are empty stand-in modules here: install only rebinds their attributes.
+    The checkpoint is the bunny_smoke run's (its key order from case_host.npz, its tensors in bunny_smoke_weights.npz)."""
     import os
     import subprocess
     import sys
     code = (
-        "import sys, yaml, torch, hydra\n"
+        "import sys, types, json, yaml, numpy as np, torch, hydra\n"
+        "from tests.helpers import GOLDEN\n"
+        "for name in ('neddf', 'neddf.render', 'neddf.network'):\n"
+        "    sys.modules[name] = types.ModuleType(name)\n"
         "import neddf_b200.install as I; I.install()\n"
-        "cfg = yaml.safe_load(open('/root/reference/pretrained/bunny_smoke/.hydra/config.yaml'))\n"
+        "cfg = yaml.safe_load(open(GOLDEN + '/bunny_smoke_config.yaml'))\n"
         "r = hydra.utils.instantiate(dict(cfg['render']), network_config=cfg['network'])\n"
         "assert type(r).__module__ == 'neddf_b200.render' and type(r.network_fine).__module__ == 'neddf_b200.network'\n"
-        "res = r.load_state_dict(torch.load('/root/reference/pretrained/bunny_smoke/models/model_02000.pth', map_location='cpu'))\n"
+        "w = np.load(GOLDEN + '/bunny_smoke_weights.npz')\n"
+        "keys = json.loads(str(np.load(GOLDEN + '/case_host.npz')['ckpt_keys']))\n"
+        "res = r.load_state_dict({k: torch.from_numpy(w[k.split('.', 1)[1]]) for k in keys})\n"
         "assert not res.missing_keys and not res.unexpected_keys\n"
         "print('ok')\n")
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join(["/root/reference", os.path.join(repo_root, "tests/golden/_refstub"), repo_root]))
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(repo_root, "tests/golden/_refstub"), repo_root]))
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
@@ -163,32 +164,34 @@ def test_vectorised_ground_truth_gather_is_bit_exact():
     assert gather_targets(item, us[:0], vs[:0], ["ColorLoss"], "cpu")["color"].shape == (0, 3)
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir("/root/reference/neddf"), reason="reference tree not present")
 def test_trainer_patch_matches_reference_method(repo_root):
     """install(patch_trainer=True) swaps BaseTrainer.construct_ground_truth for the vectorised gather;
-    the reference's own method gives the same tensors (subprocess; skimage/hydra stubbed)."""
+    it gives the tensors the reference's own method gave on the same seeded inputs (case_host.npz, recorded by
+    tests/golden/make_host_golden.py).  Subprocess; the reference's packages are empty stand-in modules."""
     import os
     import subprocess
     import sys
     code = (
         "import sys, types, numpy as np, torch\n"
-        "sk = types.ModuleType('skimage'); m = types.ModuleType('skimage.metrics')\n"
-        "m.peak_signal_noise_ratio = m.structural_similarity = None; sk.metrics = m\n"
-        "sys.modules['skimage'] = sk; sys.modules['skimage.metrics'] = m\n"
-        "from neddf.trainer.base_trainer import BaseTrainer\n"
+        "from tests.golden.make_host_golden import GATHER_KINDS, gather_inputs\n"
+        "from tests.helpers import GOLDEN\n"
+        "for name in ('neddf', 'neddf.render', 'neddf.network', 'neddf.loss', 'neddf.trainer', 'neddf.trainer.base_trainer'):\n"
+        "    sys.modules[name] = types.ModuleType(name)\n"
+        "class BaseTrainer:\n"
+        "    def construct_ground_truth(self, camera_id, us_int, vs_int, loss_types):\n"
+        "        raise NotImplementedError\n"
+        "sys.modules['neddf.trainer.base_trainer'].BaseTrainer = BaseTrainer\n"
         "ref_fn = BaseTrainer.construct_ground_truth\n"
         "import neddf_b200.install as I; I.install(patch_trainer=True)\n"
         "assert BaseTrainer.construct_ground_truth is not ref_fn\n"
-        "rng = np.random.default_rng(3)\n"
-        "class T: pass\n"
-        "t = T(); t.device = torch.device('cpu')\n"
-        "t.dataset = [dict(rgb_images=rng.integers(0, 256, (20, 30, 3), dtype=np.uint8), mask_images=rng.integers(0, 256, (20, 30), dtype=np.uint8))]\n"
-        "us = (torch.rand(64) * 29).to(torch.int16); vs = (torch.rand(64) * 19).to(torch.int16)\n"
-        "kinds = ['ColorLoss', 'MaskBCELoss', 'FieldsConstraintLoss']\n"
-        "a = ref_fn(t, 0, us, vs, kinds); b = BaseTrainer.construct_ground_truth(t, 0, us, vs, kinds)\n"
+        "rgb, mask, us, vs = gather_inputs()\n"
+        "t = types.SimpleNamespace(device=torch.device('cpu'), dataset=[dict(rgb_images=rgb, mask_images=mask)])\n"
+        "z = np.load(GOLDEN + '/case_host.npz')\n"
+        "a = {k[len('gather_'):]: torch.from_numpy(z[k]) for k in z.files if k.startswith('gather_')}\n"
+        "b = BaseTrainer.construct_ground_truth(t, 0, us, vs, GATHER_KINDS)\n"
         "assert set(a) == set(b) and all(torch.equal(a[k], b[k]) and a[k].dtype == b[k].dtype for k in a)\n"
         "print('ok')\n")
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join(["/root/reference", os.path.join(repo_root, "tests/golden/_refstub"), repo_root]))
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(repo_root, "tests/golden/_refstub"), repo_root]))
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
