@@ -355,8 +355,8 @@ int32_t neddf_dsmem_bench(int32_t mode, int32_t reps, int32_t bytes, int32_t n_c
 int32_t neddf_tc_cp_probe(int32_t lbo, int32_t sbo, uint32_t* d_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * NeRF field variant (SURVEY 8(f) item 3; neddf/network/nerf.py).  Forward only, fp32 CUDA-core kernel
- * (csrc/nerf_simt.cu): the same renderer entry points (coarse_dists, composite, sample_pdf) serve it.
+ * NeRF field variant (SURVEY 8(f) item 3; neddf/network/nerf.py).  Forward, fp32 CUDA-core kernel
+ * (csrc/nerf.cu + csrc/nerf_train_kernel.cuh): the same renderer entry points (coarse_dists, composite, sample_pdf) serve it.
  * ------------------------------------------------------------------------------------------------ */
 typedef struct neddf_nerf_config {
   int32_t embed_pos_rank;          /* nerf.py:36 (6 * rank <= 64) */
@@ -398,7 +398,7 @@ int32_t neddf_nerf_forward_rays(const neddf_nerf_t* h, const float* lowpass, con
 
 /* ------------------------------------------------------------------------------------------------
  * NeuS field variant (SURVEY 8(f) item 3; neddf/network/neus.py).  Forward only, fp32 CUDA-core kernel
- * (csrc/neus_simt.cu + csrc/neus_kernel.cuh); the normal d sdf / d position, which the reference takes with
+ * (csrc/neus_simt.cu + csrc/neus_kernel.cuh + csrc/simt_mlp.cuh); the normal d sdf / d position, which the reference takes with
  * torch.autograd.grad (neus.py:133-142), is carried forward through the SDF trunk as three Jacobian rows.
  * ------------------------------------------------------------------------------------------------ */
 typedef struct neddf_neus_config {
@@ -444,8 +444,8 @@ int32_t neddf_neus_forward_rays(const neddf_neus_t* h, const float* d_ray_dir, c
 
 /* ------------------------------------------------------------------------------------------------
  * NeRF field variant, training backward (the autograd graph of nerf.py:107-165 with respect to the parameters that
- * nerf_trainer.py:38-42 hands to Adam).  fp32 CUDA-core kernel (csrc/nerf_train.cu + csrc/nerf_train_kernel.cuh): one
- * launch recomputes the forward per 64-sample tile, walks back through the network and leaves the operands of the
+ * nerf_trainer.py:38-42 hands to Adam).  fp32 CUDA-core kernel (csrc/nerf.cu + csrc/nerf_train_kernel.cuh, the forward's tile
+ * program): one launch recomputes the forward per 64-sample tile, walks back through the network and leaves the operands of the
  * weight-gradient GEMMs in global memory; the gradients themselves are neddf_wgrad / neddf_colsum_value_rows calls on
  * those buffers (what neddf_b200/nerf.py does).  STATUS: validated by the host emulation of its tile program only
  * (tests/test_nerf_train_emul.py); opt-in in the Python layer until it has been run on hardware.

@@ -1,72 +1,54 @@
-// NeRF field variant, training backward (SURVEY 8(f) item 3): the tile program of csrc/nerf_train.cu.
+// NeRF field variant (SURVEY 8(f) item 3): the tile program of csrc/nerf.cu, forward and training backward.
 //
-// Reference: the autograd graph of NeRF.forward (neddf/network/nerf.py:107-165): position embedding with low-pass x
-// sample-size weights (:133-141), `layer_count` hidden layers with the skip concat [h | E] after the layers named in
-// `skips` (:144-148), density head + density activation (:149), colour branch Linear(width + dir embedding -> width/2),
-// ReLU, Linear(-> 3) (:96-103, :151-153).  Gradients flow to the network parameters only (what nerf_trainer.py:38-42
-// hands to Adam); sample positions carry none.
+// Reference: NeRF.forward (neddf/network/nerf.py:107-165): position embedding with low-pass x sample-size weights
+// (:133-141), `layer_count` hidden layers with the skip concat [h | E] after the layers named in `skips` (:144-148),
+// density head + density activation (:149), colour branch Linear(width + dir embedding -> width/2), ReLU,
+// Linear(-> 3) (:96-103, :151-153).  Sample geometry optionally fused like the NeDDF kernels
+// (Ray.get_sampling_points / get_sampling_cones, neddf/ray/ray.py:88-194).  Every multiply-add is an fp32 FMA (parity
+// class of the fp32 NeDDF engine) on the CUDA-core skeleton of simt_mlp.cuh.
 //
-// One kernel, per 64-sample tile: (1) recompute the forward, parking every layer's pre-activation z_l in the slot of
-// the gradient buffer G[l] and its activation h_l in X[l] (both [n][256], global, L2 resident while the tile is alive);
-// (2) walk back: g_zc1 = (Wc2^T g_color) relu'(z_c1), g_h = Wc1[:, :256]^T g_zc1 + w_density g_zd, and per hidden layer
-// g_z_l = g_h_l act'(z_l) (overwrites z_l in G[l]), g_h_{l-1} = W_l[:, :256]^T g_z_l.  The weight gradients are sums over
-// ALL samples, gW_l = X_{l-1}^T G_l: tensor-core split-K GEMMs of this library (neddf_wgrad, csrc/wgrad.cu) on the
-// buffers this kernel leaves behind; bias gradients are column sums of G_l.
-//
-// Work decomposition: the fp32 CUDA-core skeleton of csrc/nerf_simt.cu / neus_kernel.cuh (CTA of 256 threads, tile of 64
-// samples, activations K-major in shared memory, thread = 4 samples x 16 channels {4 cg + 64 i + j}, weights
-// [k padded to 16][256] through a double-buffered cp.async chunk).  The backward GEMMs are the same loop over
-// TRANSPOSED packs WT_l[k = output channel][c = input channel < 256].
-//
-// Compiled twice like neus_kernel.cuh: by nvcc into the kernel and by g++ into tests/emul (256 OS threads per CTA,
-// pthread barrier, sanitizers) - the build container has no GPU.
+// One tile program, two kernels (compile-time kTrain):
+//  - forward (kTrain = false): density and colour per sample.
+//  - training backward (kTrain = true), the autograd graph of the forward with respect to the network parameters
+//    (what nerf_trainer.py:38-42 hands to Adam; sample positions carry no gradient).  Per 64-sample tile: (1) recompute
+//    the forward, parking every layer's pre-activation z_l in the slot of the gradient buffer G[l] and its activation
+//    h_l in X[l] (both [n][256], global, L2 resident while the tile is alive); (2) walk back: g_zc1 = (Wc2^T g_color)
+//    relu'(z_c1), g_h = Wc1[:, :256]^T g_zc1 + w_density g_zd, and per hidden layer g_z_l = g_h_l act'(z_l)
+//    (overwrites z_l in G[l]), g_h_{l-1} = W_l[:, :256]^T g_z_l.  The backward GEMMs are the skeleton's loop over
+//    TRANSPOSED packs WT_l[k = output channel][c = input channel < 256].  The weight gradients are sums over ALL
+//    samples, gW_l = X_{l-1}^T G_l: tensor-core split-K GEMMs of this library (neddf_wgrad, csrc/wgrad.cu) on the
+//    buffers this kernel leaves behind; bias gradients are column sums of G_l.
 #pragma once
 
-#include "common.cuh"
-
-#ifdef __CUDACC__
-#define NERFT_LDG(p) __ldg(p)
-#else
-#define NERFT_LDG(p) (*(p))
-#endif
+#include "simt_mlp.cuh"
 
 namespace neddf {
 namespace nerft {
 
-constexpr int kT = 64;
-constexpr int kW = 256;
-constexpr int kChunk = 16;
-constexpr int kMaxE = 64;   // 6 * embed_pos_rank <= 64
-constexpr int kMaxD = 32;   // 6 * embed_dir_rank <= 32
-constexpr int kMaxLayers = 12;
-constexpr int kThreads = 256;
+using namespace simt;
+
+constexpr int kMaxE = 64;       // rows reserved for the position embedding (6 * embed_pos_rank <= 64)
+constexpr int kMaxD = 32;       // direction embedding (6 * embed_dir_rank <= 32)
+constexpr int kMaxLayers = 12;  // hidden layers
 
 enum Seg { kSegNone = 0, kSegE = 1, kSegH = 2, kSegD = 3 };
 
-struct Layer {
-  int w_off, b_off, k_pad;  // forward pack [k_pad][256] + bias [256]
-  int seg_a, n_a, seg_b, n_b;
-  int wt_off, kt_pad;       // transposed pack [kt_pad (output channels)][256 (input channels of the h part)]
-};
-
-struct Params {
-  int n_layers;                  // hidden layers; layer[n_layers] = first layer of the colour branch (128 outputs)
+struct Params : Samples {  // the samples, then:
+  // network
+  int n_layers;  // hidden layers; layer[n_layers] = first layer of the colour branch (128 outputs)
   Layer layer[kMaxLayers + 1];
-  const float* w;
+  const float* w;  // packed weights + biases (+ transposed packs for the backward)
   int embed_pos, embed_dir, n_e, n_d;
   int act, density_act;
-  int w_density_off;             // [256] + bias
-  int w_col2_off;                // [3][128] + 3 biases
+  int w_density_off;  // [256] + bias
+  int w_col2_off;     // [3][128] + 3 biases
   float lowpass[16];
-  // inputs
-  int64_t n;
-  const float *pos, *dir, *var;
-  const float *ray_dir, *ray_orig, *dists;
-  int n_edges, sampling_type;
-  float ray_radius;
-  const float* g_density;        // [n]    upstream gradient of the density output
-  const float* g_color;          // [n, 3] upstream gradient of the colour output
-  // operands of the weight-gradient GEMMs
+  // forward outputs
+  float* density;  // [n]
+  float* color;    // [n, 3]
+  // backward: upstream gradients and the operands of the weight-gradient GEMMs
+  const float* g_density;  // [n]    d loss / d density
+  const float* g_color;    // [n, 3] d loss / d colour
   float* X;    // [n_layers][n][256] activations h_l
   float* G;    // [n_layers][n][256] pre-activation gradients g_z_l (z_l between the two phases)
   float* Eo;   // [n][n_e] position embedding
@@ -82,91 +64,21 @@ constexpr int kOffD = kOffE + kMaxE * kT;
 constexpr int kOffH = kOffD + kMaxD * kT;
 constexpr int kOffW = kOffH + kW * kT;
 constexpr int kOffGeo = kOffW + 2 * kChunk * kW;  // [kT][9] pos, dir, var
-constexpr int kOffUp = kOffGeo + kT * 9;          // [kT][4] g_color (3), g_zd
+constexpr int kOffUp = kOffGeo + kT * 9;          // [kT][4] g_color (3), g_zd (backward only)
 constexpr int kSmemFloats = kOffUp + kT * 4;
 constexpr size_t kSmemBytes = (size_t)kSmemFloats * sizeof(float);
 
-// value and slope of the plain activations of nerf.py:72-81 (torch.relu / leaky_relu(0.01) and their autograd slopes,
-// tanhExp of nn_module/tanh_exp.py:26-31 with its backward :57-60)
-__device__ __forceinline__ void act_fd(int act, float x, float& y, float& d1) {
-  if (act == NEDDF_ACT_TANHEXP) {
-    const float ex = expf(x);
-    const float tx = tanhf(ex);
-    y = x * tx;
-    d1 = tx - x * ex * (tx * tx - 1.0f);
-    if (x > 20.0f) {
-      y = x;
-      d1 = 1.0f;
-    }
-  } else if (act == NEDDF_ACT_RELU) {
-    d1 = (x > 0.0f) ? 1.0f : 0.0f;
-    y = (x > 0.0f) ? x : 0.0f;
-  } else {
-    d1 = (x > 0.0f) ? 1.0f : 0.01f;
-    y = x * d1;
-  }
-}
-
-__device__ __forceinline__ const float* seg_ptr(const float* smem, int seg) {
+__device__ __forceinline__ float* seg_ptr(float* smem, int seg) {
   return smem + (seg == kSegE ? kOffE : (seg == kSegD ? kOffD : kOffH));
 }
 
-// acc[i][j][s] = sum_k W[k][4 cg + 64 i + j] * seg[k][4 sg + s]; same entry / exit contract as neus::layer_gemm
 template <class Ctx>
-__device__ __forceinline__ void gemm(Ctx& cx, const float* wl, int k_pad, int seg_a, int n_a, int seg_b, int n_b, float* smem,
-                                     float (&acc)[4][4][4]) {
-  const int tid = cx.tid;
-  const int cg = tid & 15, sg = tid >> 4;
-  const float* A = seg_ptr(smem, seg_a);
-  const float* B = seg_ptr(smem, seg_b);
-  float* Wc = smem + kOffW;
-  const int n_chunks = k_pad / kChunk;
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-#pragma unroll
-      for (int s = 0; s < 4; ++s) acc[i][j][s] = 0.f;
-  auto load_chunk = [&](int buf, int c) {
-    const float* src = wl + (size_t)c * kChunk * kW;
-    float* dst = Wc + buf * kChunk * kW;
-#pragma unroll
-    for (int u = 0; u < (kChunk * kW / 4) / kThreads; ++u) cx.cp16(dst + 4 * (tid + u * kThreads), src + 4 * (tid + u * kThreads));
-    cx.cp_commit();
-  };
-  load_chunk(0, 0);
-  for (int c = 0; c < n_chunks; ++c) {
-    if (c + 1 < n_chunks) {
-      load_chunk((c + 1) & 1, c + 1);
-      cx.cp_wait_1();
-    } else {
-      cx.cp_wait_0();
-    }
-    cx.sync();
-    const float* wc = Wc + (c & 1) * kChunk * kW;
-#pragma unroll 4
-    for (int kk = 0; kk < kChunk; ++kk) {
-      const int k = c * kChunk + kk;
-      const float* rowp = (k < n_a) ? A + k * kT : ((k < n_a + n_b) ? B + (k - n_a) * kT : A);
-      const float4 a = *reinterpret_cast<const float4*>(rowp + 4 * sg);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float4 w4 = *reinterpret_cast<const float4*>(wc + kk * kW + 4 * cg + 64 * i);
-        const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          acc[i][j][0] = fmaf(wv[j], a.x, acc[i][j][0]);
-          acc[i][j][1] = fmaf(wv[j], a.y, acc[i][j][1]);
-          acc[i][j][2] = fmaf(wv[j], a.z, acc[i][j][2]);
-          acc[i][j][3] = fmaf(wv[j], a.w, acc[i][j][3]);
-        }
-      }
-    }
-    cx.sync();
-  }
+__device__ __forceinline__ void gemm(Ctx& cx, const float* w, const Layer& Ly, float* smem, float (&acc)[4][4][4]) {
+  layer_gemm(cx, w + Ly.w_off, Ly.k_pad, seg_ptr(smem, Ly.seg_a), Ly.n_a, seg_ptr(smem, Ly.seg_b), Ly.n_b, smem + kOffW, acc);
 }
 
-template <class Ctx>
+// One CTA: tiles cx.block, cx.block + cx.nblocks, ...
+template <bool kTrain = true, class Ctx>
 __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* smem) {
   float* E = smem + kOffE;
   float* D = smem + kOffD;
@@ -175,49 +87,29 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
   float* up = smem + kOffUp;
   const int tid = cx.tid;
   const int cg = tid & 15, sg = tid >> 4;
-  const int64_t n_tiles = (P.n + kT - 1) / kT;
+  const int64_t N = P.n;
+  const int64_t n_tiles = (N + kT - 1) / kT;
   const int L = P.n_layers;
   float acc[4][4][4];
 
   for (int64_t tile = cx.block; tile < n_tiles; tile += cx.nblocks) {
     const int64_t n0 = tile * kT;
-    // ---- geometry + upstream gradients of the tile's samples (one thread per sample) ----
+    // ---- geometry (+ upstream gradients) of the tile's samples (one thread per sample) ----
     if (tid < kT) {
-      float pos[3] = {0.f, 0.f, 0.f}, dir[3] = {0.f, 0.f, 1.f}, var[3] = {0.f, 0.f, 0.f};
-      float gc[3] = {0.f, 0.f, 0.f}, gd = 0.f;
+      float pos[3], dir[3], var[3];
       const int64_t n = n0 + tid;
-      if (n < P.n) {
-        if (P.dists) {
-          const int64_t b = n / P.n_edges;
-          const int j = (int)(n - b * P.n_edges);
-          const float* row = P.dists + b * P.n_edges;
-          float o[3];
-#pragma unroll
-          for (int i = 0; i < 3; ++i) {
-            o[i] = P.ray_orig[3 * b + i];
-            dir[i] = P.ray_dir[3 * b + i];
-          }
-          sample_geometry(P.sampling_type, P.ray_radius, o, dir, row[j], far_edge(row, j, P.n_edges), pos, var);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 3; ++i) {
-            pos[i] = P.pos[3 * n + i];
-            dir[i] = P.dir[3 * n + i];
-            var[i] = P.var[3 * n + i];
-          }
-        }
-#pragma unroll
-        for (int i = 0; i < 3; ++i) gc[i] = P.g_color[3 * n + i];
-        gd = P.g_density[n];
-      }
+      load_sample(P, n, pos, dir, var);
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
         geo[tid * 9 + i] = pos[i];
         geo[tid * 9 + 3 + i] = dir[i];
         geo[tid * 9 + 6 + i] = var[i];
-        up[tid * 4 + i] = gc[i];
       }
-      up[tid * 4 + 3] = gd;  // g_density for now; becomes g_zd after the density head
+      if constexpr (kTrain) {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) up[tid * 4 + i] = (n < N) ? P.g_color[3 * n + i] : 0.f;
+        up[tid * 4 + 3] = (n < N) ? P.g_density[n] : 0.f;  // g_density for now; becomes g_zd after the density head
+      }
     }
     cx.sync();
     // ---- embeddings (nerf.py:133-142): four threads per sample ----
@@ -243,162 +135,169 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
       }
     }
     cx.sync();
-    // embeddings as GEMM operands of the weight gradients: [n][n_e], [n][n_d]
-    for (int idx = tid; idx < kT * P.n_e; idx += kThreads) {
-      const int s = idx / P.n_e, k = idx - s * P.n_e;
-      if (n0 + s < P.n) P.Eo[(n0 + s) * P.n_e + k] = E[k * kT + s];
-    }
-    for (int idx = tid; idx < kT * P.n_d; idx += kThreads) {
-      const int s = idx / P.n_d, k = idx - s * P.n_d;
-      if (n0 + s < P.n) P.Do[(n0 + s) * P.n_d + k] = D[k * kT + s];
+    if constexpr (kTrain) {  // embeddings as GEMM operands of the weight gradients: [n][n_e], [n][n_d]
+      for (int idx = tid; idx < kT * P.n_e; idx += kThreads) {
+        const int s = idx / P.n_e, k = idx - s * P.n_e;
+        if (n0 + s < N) P.Eo[(n0 + s) * P.n_e + k] = E[k * kT + s];
+      }
+      for (int idx = tid; idx < kT * P.n_d; idx += kThreads) {
+        const int s = idx / P.n_d, k = idx - s * P.n_d;
+        if (n0 + s < N) P.Do[(n0 + s) * P.n_d + k] = D[k * kT + s];
+      }
     }
 
-    // ================================ phase 1: forward, parking z_l and h_l ================================
-    for (int l = 0; l < L; ++l) {
+    // ---- hidden layers (nerf.py:144-148), then the colour branch's first layer (nerf.py:96-100, :151-152) ----
+    for (int l = 0; l <= L; ++l) {
+      if (l == L && tid < kT) {
+        // density head (nerf.py:149) on the trunk's features, before the colour layer overwrites H;
+        // the backward's g_zd = g_density * act'(z_d)
+        const float* wd = P.w + P.w_density_off;
+        const int64_t n = n0 + tid;
+        float zd = LDG(wd + kW);
+        for (int c = 0; c < kW; ++c) zd = fmaf(LDG(wd + c), H[c * kT + tid], zd);
+        if constexpr (kTrain) {
+          float y, d1;
+          act_fd(P.density_act, zd, y, d1);
+          const float gzd = up[tid * 4 + 3] * d1;
+          up[tid * 4 + 3] = gzd;
+          if (n < N) P.GZD[n] = gzd;
+        } else {
+          if (n < N) P.density[n] = density_act(P.density_act, zd);
+        }
+        // (no barrier: the layer below starts by reading H, writes it and reads `up` only after its own barriers)
+      }
       const Layer& Ly = P.layer[l];
-      gemm(cx, P.w + Ly.w_off, Ly.k_pad, Ly.seg_a, Ly.n_a, Ly.seg_b, Ly.n_b, smem, acc);
+      gemm(cx, P.w, Ly, smem, acc);
+      const int act = (l < L) ? P.act : NEDDF_ACT_RELU;  // outL_color's nn.ReLU (nerf.py:99)
       const float* bl = P.w + Ly.b_off;
-      float* Xl = P.X + (size_t)l * P.n * kW;
-      float* Gl = P.G + (size_t)l * P.n * kW;
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         const int ch0 = 4 * cg + 64 * i;
-        const float4 b4 = make_float4(NERFT_LDG(bl + ch0), NERFT_LDG(bl + ch0 + 1), NERFT_LDG(bl + ch0 + 2), NERFT_LDG(bl + ch0 + 3));
-        const float bb[4] = {b4.x, b4.y, b4.z, b4.w};
         float z[4][4], h[4][4];  // [j][s]
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
+        for (int j = 0; j < 4; ++j) {
+          const float b = LDG(bl + ch0 + j);
 #pragma unroll
           for (int s = 0; s < 4; ++s) {
             float d1;
-            z[j][s] = acc[i][j][s] + bb[j];
-            act_fd(P.act, z[j][s], h[j][s], d1);
+            z[j][s] = acc[i][j][s] + b;
+            act_fd(act, z[j][s], h[j][s], d1);
           }
+        }
+        if constexpr (kTrain) {
+          if (l < L) {  // park z_l and h_l
+            float* Xl = P.X + (size_t)l * N * kW;
+            float* Gl = P.G + (size_t)l * N * kW;
+#pragma unroll
+            for (int s = 0; s < 4; ++s) {
+              const int64_t n = n0 + 4 * sg + s;
+              if (n < N) {
+                *reinterpret_cast<float4*>(Gl + n * kW + ch0) = make_float4(z[0][s], z[1][s], z[2][s], z[3][s]);
+                *reinterpret_cast<float4*>(Xl + n * kW + ch0) = make_float4(h[0][s], h[1][s], h[2][s], h[3][s]);
+              }
+            }
+          } else {  // z becomes g_zc1 = (Wc2^T g_color) relu'(z_c1), which H carries into the backward
+            const float* wc2 = P.w + P.w_col2_off;  // [3][128]
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const int ch = ch0 + j;
+              const bool live = ch < kW / 2;  // the colour branch is 128 wide; the padded half stays zero
+              const float w0 = live ? LDG(wc2 + ch) : 0.f;
+              const float w1 = live ? LDG(wc2 + kW / 2 + ch) : 0.f;
+              const float w2 = live ? LDG(wc2 + kW + ch) : 0.f;
+#pragma unroll
+              for (int s = 0; s < 4; ++s) {
+                const float* g = up + (4 * sg + s) * 4;
+                z[j][s] = (z[j][s] > 0.f) ? fmaf(w2, g[2], fmaf(w1, g[1], w0 * g[0])) : 0.f;
+              }
+            }
+#pragma unroll
+            for (int s = 0; s < 4; ++s) {
+              const int64_t n = n0 + 4 * sg + s;
+              if (n < N) {
+                *reinterpret_cast<float4*>(P.C1 + n * kW + ch0) = make_float4(h[0][s], h[1][s], h[2][s], h[3][s]);
+                *reinterpret_cast<float4*>(P.GC1 + n * kW + ch0) = make_float4(z[0][s], z[1][s], z[2][s], z[3][s]);
+              }
+            }
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+#pragma unroll
+              for (int s = 0; s < 4; ++s) h[j][s] = z[j][s];
+          }
+        }
 #pragma unroll
         for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(H + (ch0 + j) * kT + 4 * sg) = make_float4(h[j][0], h[j][1], h[j][2], h[j][3]);
-#pragma unroll
-        for (int s = 0; s < 4; ++s) {
-          const int64_t n = n0 + 4 * sg + s;
-          if (n < P.n) {
-            *reinterpret_cast<float4*>(Gl + n * kW + ch0) = make_float4(z[0][s], z[1][s], z[2][s], z[3][s]);
-            *reinterpret_cast<float4*>(Xl + n * kW + ch0) = make_float4(h[0][s], h[1][s], h[2][s], h[3][s]);
-          }
-        }
       }
       cx.sync();
     }
-    // ---- density head (nerf.py:149) and its gradient: g_zd = g_density * act'(z_d) ----
-    if (tid < kT) {
-      const float* wd = P.w + P.w_density_off;
-      float zd = NERFT_LDG(wd + kW);
-      for (int c = 0; c < kW; ++c) zd = fmaf(NERFT_LDG(wd + c), H[c * kT + tid], zd);
-      float y, d1;
-      act_fd(P.density_act, zd, y, d1);
-      const float gzd = up[tid * 4 + 3] * d1;
-      up[tid * 4 + 3] = gzd;
-      if (n0 + tid < P.n) P.GZD[n0 + tid] = gzd;
-    }
-    // (no barrier: `up` is next read behind the barriers of the colour layer's GEMM)
-    // ---- colour branch, first layer (nerf.py:96-100, :151-152) + gradient of its pre-activation ----
-    {
-      const Layer& Ly = P.layer[L];
-      gemm(cx, P.w + Ly.w_off, Ly.k_pad, Ly.seg_a, Ly.n_a, Ly.seg_b, Ly.n_b, smem, acc);
-      const float* bl = P.w + Ly.b_off;
-      const float* wc2 = P.w + P.w_col2_off;  // [3][128]
+
+    if constexpr (!kTrain) {
+      // ---- colour output (nerf.py:101-102): 3 x (width / 2) ----
+      if (tid < kT) {
+        const float* wc2 = P.w + P.w_col2_off;
+        const int64_t n = n0 + tid;
+        float o[3];
 #pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int ch0 = 4 * cg + 64 * i;
-        float c1[4][4], gz[4][4];  // [j][s]
+        for (int c = 0; c < 3; ++c) {
+          float a = wc2[3 * (kW / 2) + c];
+          for (int k = 0; k < kW / 2; ++k) a = fmaf(LDG(wc2 + c * (kW / 2) + k), H[k * kT + tid], a);
+          o[c] = a;
+        }
+        if (n < N) {
+          P.color[3 * n + 0] = o[0];
+          P.color[3 * n + 1] = o[1];
+          P.color[3 * n + 2] = o[2];
+        }
+      }
+      cx.sync();  // H, E, D, geo are rewritten by the next tile
+    } else {
+      // ---- backward through the trunk ----
+      // H holds the gradient of the pre-activation of the layer ABOVE (k = its output channel); step l turns it into
+      // g_z_l = (W_above[:, :256]^T g_z_above [+ w_density g_zd for the last hidden layer]) act'(z_l).
+      for (int l = L - 1; l >= 0; --l) {
+        const Layer& Up = P.layer[l + 1];  // l + 1 == L: the colour branch's first layer (128 outputs)
+        layer_gemm(cx, P.w + Up.wt_off, Up.kt_pad, H, Up.kt_pad, H, 0, smem + kOffW, acc);
+        float* Gl = P.G + (size_t)l * N * kW;
+        const float* wd = P.w + P.w_density_off;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int ch = ch0 + j;
-          const bool live = ch < kW / 2;  // the colour branch is 128 wide; the padded half stays zero
-          const float b = NERFT_LDG(bl + ch);
-          const float w0 = live ? NERFT_LDG(wc2 + ch) : 0.f;
-          const float w1 = live ? NERFT_LDG(wc2 + kW / 2 + ch) : 0.f;
-          const float w2 = live ? NERFT_LDG(wc2 + kW + ch) : 0.f;
+        for (int i = 0; i < 4; ++i) {
+          const int ch0 = 4 * cg + 64 * i;
+          float gz[4][4];  // [j][s]
+          float wdj[4] = {0.f, 0.f, 0.f, 0.f};
+          if (l == L - 1) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) wdj[j] = LDG(wd + ch0 + j);
+          }
 #pragma unroll
           for (int s = 0; s < 4; ++s) {
-            const float z = acc[i][j][s] + b;
-            const float* g = up + (4 * sg + s) * 4;
-            c1[j][s] = (z > 0.f) ? z : 0.f;                                          // nn.ReLU (nerf.py:99)
-            gz[j][s] = (z > 0.f) ? fmaf(w2, g[2], fmaf(w1, g[1], w0 * g[0])) : 0.f;  // (Wc2^T g_color) relu'(z)
-          }
-        }
+            const int64_t n = n0 + 4 * sg + s;
+            float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (n < N) z4 = *reinterpret_cast<const float4*>(Gl + n * kW + ch0);  // z_l parked by the forward
+            const float zz[4] = {z4.x, z4.y, z4.z, z4.w};
+            const float gzd = up[(4 * sg + s) * 4 + 3];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(H + (ch0 + j) * kT + 4 * sg) = make_float4(gz[j][0], gz[j][1], gz[j][2], gz[j][3]);
-#pragma unroll
-        for (int s = 0; s < 4; ++s) {
-          const int64_t n = n0 + 4 * sg + s;
-          if (n < P.n) {
-            *reinterpret_cast<float4*>(P.C1 + n * kW + ch0) = make_float4(c1[0][s], c1[1][s], c1[2][s], c1[3][s]);
-            *reinterpret_cast<float4*>(P.GC1 + n * kW + ch0) = make_float4(gz[0][s], gz[1][s], gz[2][s], gz[3][s]);
+            for (int j = 0; j < 4; ++j) {
+              float y, d1;
+              act_fd(P.act, zz[j], y, d1);
+              gz[j][s] = fmaf(wdj[j], gzd, acc[i][j][s]) * d1;
+            }
+            if (n < N) *reinterpret_cast<float4*>(Gl + n * kW + ch0) = make_float4(gz[0][s], gz[1][s], gz[2][s], gz[3][s]);
           }
+#pragma unroll
+          for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(H + (ch0 + j) * kT + 4 * sg) = make_float4(gz[j][0], gz[j][1], gz[j][2], gz[j][3]);
         }
+        cx.sync();
       }
-      cx.sync();
+      // (the trailing barrier of the last step also protects E, D, H, geo, up against the next tile)
     }
-
-    // ================================ phase 2: backward through the trunk ================================
-    // H holds the gradient of the pre-activation of the layer ABOVE (k = its output channel); step l turns it into
-    // g_z_l = (W_above[:, :256]^T g_z_above [+ w_density g_zd for the last hidden layer]) act'(z_l).
-    for (int l = L - 1; l >= 0; --l) {
-      const Layer& Up = P.layer[l + 1];  // l + 1 == L: the colour branch's first layer (128 outputs)
-      gemm(cx, P.w + Up.wt_off, Up.kt_pad, kSegH, Up.kt_pad, kSegNone, 0, smem, acc);
-      float* Gl = P.G + (size_t)l * P.n * kW;
-      const float* wd = P.w + P.w_density_off;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int ch0 = 4 * cg + 64 * i;
-        float gz[4][4];  // [j][s]
-        float wdj[4] = {0.f, 0.f, 0.f, 0.f};
-        if (l == L - 1) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) wdj[j] = NERFT_LDG(wd + ch0 + j);
-        }
-#pragma unroll
-        for (int s = 0; s < 4; ++s) {
-          const int64_t n = n0 + 4 * sg + s;
-          float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (n < P.n) z4 = *reinterpret_cast<const float4*>(Gl + n * kW + ch0);  // z_l parked by phase 1
-          const float zz[4] = {z4.x, z4.y, z4.z, z4.w};
-          const float gzd = up[(4 * sg + s) * 4 + 3];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            float y, d1;
-            act_fd(P.act, zz[j], y, d1);
-            gz[j][s] = fmaf(wdj[j], gzd, acc[i][j][s]) * d1;
-          }
-          if (n < P.n) *reinterpret_cast<float4*>(Gl + n * kW + ch0) = make_float4(gz[0][s], gz[1][s], gz[2][s], gz[3][s]);
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) *reinterpret_cast<float4*>(H + (ch0 + j) * kT + 4 * sg) = make_float4(gz[j][0], gz[j][1], gz[j][2], gz[j][3]);
-      }
-      cx.sync();
-    }
-    // (the trailing barrier of the last step also protects E, D, H, geo, up against the next tile)
   }
-}
-
-// torch Linear weight [out][in] -> entry (k, c) of the forward pack [in padded][256]
-__device__ __forceinline__ float pack_fwd(const float* w, int n_in, int n_out, int k, int c) {
-  return (k < n_in && c < n_out) ? w[(size_t)c * n_in + k] : 0.f;
-}
-// ... -> entry (k, c) of the transposed pack [out padded][256]: the first 256 input channels (the h part) of row k
-__device__ __forceinline__ float pack_bwd(const float* w, int n_in, int n_out, int k, int c) {
-  return (k < n_out && c < n_in && c < kW) ? w[(size_t)k * n_in + c] : 0.f;
 }
 
 // ---------------------------------------------------------------------------------------------
 // host: layer table (nerf.py:86-103)
 // ---------------------------------------------------------------------------------------------
-inline bool is_skip(const neddf_nerf_config_t* c, int lid) {
-  for (int i = 0; i < c->n_skips; ++i)
-    if (c->skips[i] == lid) return true;
-  return false;
-}
 
-// layers.0 .. layers.{L-1}, outL_density, outL_color.0, outL_color.2
+// layers.0 .. layers.{L-1}, outL_density, outL_color.0, outL_color.2; returns the count
 inline int layer_shapes(const neddf_nerf_config_t* c, int* sin, int* sout) {
   const int in_pos = 6 * c->embed_pos_rank, in_dir = 6 * c->embed_dir_rank, W = c->layer_width;
   int n = 0;
@@ -413,20 +312,26 @@ inline int layer_shapes(const neddf_nerf_config_t* c, int* sin, int* sout) {
   return n;
 }
 
-inline const char* unsupported(const neddf_nerf_config_t* c) {
-  if (c->layer_width != kW) return "layer_width must be 256";
-  if (c->layer_count < 2 || c->layer_count > kMaxLayers) return "layer_count must be 2..12";
-  if (c->embed_pos_rank < 1 || 6 * c->embed_pos_rank > kMaxE || c->embed_pos_rank > 16) return "6 * embed_pos_rank must be <= 64";
-  if (c->embed_dir_rank < 1 || 6 * c->embed_dir_rank > kMaxD) return "6 * embed_dir_rank must be <= 32";
-  if (c->n_skips < 0 || c->n_skips > 8) return "at most 8 skips";
+// NULL = supported, else the reason and in *code (if given) NEDDF_E_INVALID (malformed) or NEDDF_E_UNSUPPORTED (not covered)
+inline const char* unsupported(const neddf_nerf_config_t* c, int32_t* code = nullptr) {
+  int32_t unused;
+  if (!code) code = &unused;
+  *code = NEDDF_E_INVALID;
+  if (c->n_skips < 0 || c->n_skips > 8) return "bad skips";
   for (int a : {c->activation_type, c->density_activation_type})
     if (a != NEDDF_ACT_TANHEXP && a != NEDDF_ACT_RELU && a != NEDDF_ACT_LEAKYRELU) return "bad activation";
+  *code = NEDDF_E_UNSUPPORTED;
+  if (c->layer_width != kW) return "layer_width must be 256";
+  if (c->layer_count < 2 || c->layer_count > kMaxLayers) return "layer_count must be 2..12";
+  if (c->embed_pos_rank < 1 || 6 * c->embed_pos_rank > kMaxE || c->embed_dir_rank < 1 || 6 * c->embed_dir_rank > kMaxD)
+    return "embedding ranks must satisfy 6 pos <= 64, 6 dir <= 32";
   if (is_skip(c, c->layer_count - 1)) return "a skip after the last hidden layer widens the heads (not covered)";
   return nullptr;
 }
 
-// fills the network part of P; returns the floats of the packed weight buffer
-inline size_t build_program(const neddf_nerf_config_t* c, Params& P) {
+// fills the network part of P; `backward` adds the transposed packs the training kernel reads.  Returns the floats of
+// weight buffer.
+inline size_t build_program(const neddf_nerf_config_t* c, Params& P, bool backward = true) {
   const int L = c->layer_count;
   P.n_layers = L;
   P.embed_pos = c->embed_pos_rank;
@@ -436,16 +341,16 @@ inline size_t build_program(const neddf_nerf_config_t* c, Params& P) {
   P.act = c->activation_type;
   P.density_act = c->density_activation_type;
   size_t off = 0;
-  auto pad16 = [](int k) { return (k + kChunk - 1) / kChunk * kChunk; };
   for (int l = 0; l <= L; ++l) {
     Layer& Ly = P.layer[l];
     if (l == 0) { Ly.seg_a = kSegE; Ly.n_a = P.n_e; Ly.seg_b = kSegNone; Ly.n_b = 0; }
     else if (l < L) { Ly.seg_a = kSegH; Ly.n_a = kW; Ly.seg_b = is_skip(c, l - 1) ? kSegE : kSegNone; Ly.n_b = Ly.seg_b ? P.n_e : 0; }
     else { Ly.seg_a = kSegH; Ly.n_a = kW; Ly.seg_b = kSegD; Ly.n_b = P.n_d; }
-    Ly.k_pad = pad16(Ly.n_a + Ly.n_b);
+    Ly.k_pad = (Ly.n_a + Ly.n_b + kChunk - 1) / kChunk * kChunk;
     Ly.w_off = (int)off; off += (size_t)Ly.k_pad * kW;
     Ly.b_off = (int)off; off += kW;
-    Ly.kt_pad = (l == 0) ? 0 : ((l < L) ? kW : kW / 2);  // layer 0 has nothing below it to propagate to
+    // layer 0 has nothing below it to propagate to
+    Ly.kt_pad = (!backward || l == 0) ? 0 : ((l < L) ? kW : kW / 2);
     Ly.wt_off = (int)off; off += (size_t)Ly.kt_pad * kW;
   }
   P.w_density_off = (int)off; off += kW + 4;

@@ -11,52 +11,34 @@
 // (value, d/dx, d/dy, d/dz; the layout of the NeDDF kernels), G = f'(x) (J W) - the same number as the reference's
 // reverse-mode gradient up to rounding (oracle.neus_forward_jac against oracle.neus_forward, tests/test_neus_oracle.py).
 //
-// Work decomposition (the fp32 CUDA-core skeleton of csrc/nerf_simt.cu)
+// Work decomposition (the fp32 CUDA-core skeleton of simt_mlp.cuh)
 //   CTA (256 threads) = tile of 64 samples, persistent over tiles.  Activations K-major in shared memory
 //   (row = channel, 64 columns).  SDF trunk: four passes over sub-tiles of 16 samples, column = 4 sample + row type;
 //   the last SDF layer parks its value rows in F (column = sample) and the normal in the colour input head X.
 //   Colour trunk: one pass over the 64 samples (value rows only), input rows "X then F", hidden rows in H.
 //   Thread (cg = tid % 16, sg = tid / 16) owns columns 4 sg .. 4 sg + 3 (SDF trunk: the four row types of sample
 //   sg; colour trunk: four samples) and the 16 output channels {4 cg + 64 i + j}.
-//   Weights: [in rows padded to 16][256] fp32, streamed through a double-buffered 16-row chunk (cp.async).
 //
-// This header is compiled twice: by nvcc into the kernel (Ctx = the CUDA thread) and by g++ into
-// tests/emul/libneus_emul.so (Ctx = one of 256 OS threads per CTA, a barrier for __syncthreads) so that the very
-// same index arithmetic is checked against the goldens in the build container, which has no GPU.
+// Compiled twice like simt_mlp.cuh: by nvcc into the kernel and by g++ into tests/emul/libneus_emul.so, where it is
+// checked against the goldens.
 #pragma once
 
-#include "common.cuh"
-
-#ifdef __CUDACC__
-#define NEUS_LDG(p) __ldg(p)
-#else
-#define NEUS_LDG(p) (*(p))
-#endif
+#include "simt_mlp.cuh"
 
 namespace neddf {
 namespace neus {
 
-constexpr int kT = 64;       // samples per tile
+using namespace simt;
+
 constexpr int kSub = 16;     // samples per SDF sub-tile (4 columns each)
-constexpr int kW = 256;      // layer width (fixed)
-constexpr int kChunk = 16;   // weight rows per shared-memory chunk
 constexpr int kMaxE = 64;    // rows reserved for the position embedding (6 * rank <= 64)
 constexpr int kMaxX = 32;    // colour input head [pos 3 | dir embedding 6 * rank | normal 3] (<= 32 rows)
 constexpr int kMaxSdf = 12;  // SDF layers
 constexpr int kMaxCol = 12;  // colour layers of width 256 (the 3-channel output layer is a per-sample head)
-constexpr int kThreads = 256;
 
 enum Seg { kSegNone = 0, kSegE = 1, kSegH = 2, kSegX = 3, kSegF = 4 };
 
-struct Layer {
-  int w_off;       // float offset of the packed [k_pad][256] block
-  int b_off;       // float offset of the [256] bias block
-  int k_pad;       // input rows padded to a multiple of kChunk
-  int seg_a, n_a;  // first input segment and its rows
-  int seg_b, n_b;  // second one (kSegNone: none)
-};
-
-struct Params {
+struct Params : Samples {  // the samples (var unused: the NeuS embeddings are plain), then:
   // network
   int n_sdf, n_col;
   Layer lsdf[kMaxSdf];
@@ -66,12 +48,6 @@ struct Params {
   int embed_pos, embed_dir;
   int act;       // NEDDF_ACT_RELU | NEDDF_ACT_TANHEXP
   const float* w;
-  // inputs: explicit samples or rays + edges
-  int64_t n;
-  const float *pos, *dir;
-  const float *ray_dir, *ray_orig, *dists;
-  int n_edges, sampling_type;
-  float ray_radius;
   // outputs ([n], [n], [n,3], optional [n,3])
   float* sdf;
   float* density;
@@ -90,24 +66,6 @@ constexpr int kOffSdf = kOffGeo + kT * 6;         // [kT] sdf of the tile's samp
 constexpr int kSmemFloats = kOffSdf + kT;
 constexpr size_t kSmemBytes = (size_t)kSmemFloats * sizeof(float);
 
-// Activation with first derivative.  ReLU: torch.relu and its autograd slope (x > 0); tanhExp: nn_module/tanh_exp.py
-// :26-31 forward, :57-60 backward (d = tx - x ex (tx^2 - 1), 1 above the threshold).
-__device__ __forceinline__ void act_fd(int act, float x, float& y, float& d1) {
-  if (act == NEDDF_ACT_TANHEXP) {
-    const float ex = expf(x);
-    const float tx = tanhf(ex);
-    y = x * tx;
-    d1 = tx - x * ex * (tx * tx - 1.0f);
-    if (x > 20.0f) {
-      y = x;
-      d1 = 1.0f;
-    }
-  } else {
-    d1 = (x > 0.0f) ? 1.0f : 0.0f;
-    y = (x > 0.0f) ? x : 0.0f;
-  }
-}
-
 // neus.py:150-153, one rounding per torch op
 __device__ __forceinline__ float sdf_density(float sdf, float variance) {
   const float v10 = __fmul_rn(variance, 10.0f);
@@ -116,66 +74,13 @@ __device__ __forceinline__ float sdf_density(float sdf, float variance) {
   return __fmul_rn(__fmul_rn(v10, ex), __frcp_rn(__fmul_rn(onep, onep)));
 }
 
-__device__ __forceinline__ const float* seg_ptr(const float* smem, int seg) {
+__device__ __forceinline__ float* seg_ptr(float* smem, int seg) {
   return smem + (seg == kSegE ? kOffE : (seg == kSegX ? kOffX : (seg == kSegF ? kOffF : kOffH)));
 }
 
-// acc[i][j][col] = sum_k W[k][4 cg + 64 i + j] * act[k][4 sg + col] over the layer's input rows.
-// Entry: every thread has passed a barrier after the last write to the input segments and after the last read of
-// the weight chunk buffers.  Exit: every thread has finished reading the input segments (trailing barrier).
 template <class Ctx>
-__device__ __forceinline__ void layer_gemm(Ctx& cx, const Params& P, const Layer& L, float* smem, float (&acc)[4][4][4]) {
-  const int tid = cx.tid;
-  const int cg = tid & 15, sg = tid >> 4;
-  const float* A = seg_ptr(smem, L.seg_a);
-  const float* B = seg_ptr(smem, L.seg_b);
-  const float* wl = P.w + L.w_off;
-  float* Wc = smem + kOffW;
-  const int n_chunks = L.k_pad / kChunk;
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-#pragma unroll
-      for (int s = 0; s < 4; ++s) acc[i][j][s] = 0.f;
-  auto load_chunk = [&](int buf, int c) {
-    const float* src = wl + (size_t)c * kChunk * kW;
-    float* dst = Wc + buf * kChunk * kW;
-#pragma unroll
-    for (int u = 0; u < (kChunk * kW / 4) / kThreads; ++u) cx.cp16(dst + 4 * (tid + u * kThreads), src + 4 * (tid + u * kThreads));
-    cx.cp_commit();
-  };
-  load_chunk(0, 0);
-  for (int c = 0; c < n_chunks; ++c) {
-    if (c + 1 < n_chunks) {
-      load_chunk((c + 1) & 1, c + 1);
-      cx.cp_wait_1();
-    } else {
-      cx.cp_wait_0();
-    }
-    cx.sync();
-    const float* wc = Wc + (c & 1) * kChunk * kW;
-#pragma unroll 4
-    for (int kk = 0; kk < kChunk; ++kk) {
-      const int k = c * kChunk + kk;
-      // rows beyond the layer's inputs carry zero weights; they read row 0 of the first segment
-      const float* rowp = (k < L.n_a) ? A + k * kT : ((k < L.n_a + L.n_b) ? B + (k - L.n_a) * kT : A);
-      const float4 a = *reinterpret_cast<const float4*>(rowp + 4 * sg);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float4 w4 = *reinterpret_cast<const float4*>(wc + kk * kW + 4 * cg + 64 * i);
-        const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          acc[i][j][0] = fmaf(wv[j], a.x, acc[i][j][0]);
-          acc[i][j][1] = fmaf(wv[j], a.y, acc[i][j][1]);
-          acc[i][j][2] = fmaf(wv[j], a.z, acc[i][j][2]);
-          acc[i][j][3] = fmaf(wv[j], a.w, acc[i][j][3]);
-        }
-      }
-    }
-    cx.sync();  // chunk buffer free; after the last chunk: every thread is done reading the input segments
-  }
+__device__ __forceinline__ void gemm(Ctx& cx, const Params& P, const Layer& L, float* smem, float (&acc)[4][4][4]) {
+  layer_gemm(cx, P.w + L.w_off, L.k_pad, seg_ptr(smem, L.seg_a), L.n_a, seg_ptr(smem, L.seg_b), L.n_b, smem + kOffW, acc);
 }
 
 // One CTA: tiles cx.block, cx.block + cx.nblocks, ...
@@ -199,28 +104,8 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
     const int64_t n0 = tile * kT;
     // ---- geometry of the tile's samples (one thread per sample); rows 0..2 of X = position (neus.py:145) ----
     if (tid < kT) {
-      float pos[3] = {0.f, 0.f, 0.f}, dir[3] = {0.f, 0.f, 1.f}, var[3];
-      const int64_t n = n0 + tid;
-      if (n < P.n) {
-        if (P.dists) {
-          const int64_t b = n / P.n_edges;
-          const int j = (int)(n - b * P.n_edges);
-          const float* row = P.dists + b * P.n_edges;
-          float o[3];
-#pragma unroll
-          for (int i = 0; i < 3; ++i) {
-            o[i] = P.ray_orig[3 * b + i];
-            dir[i] = P.ray_dir[3 * b + i];
-          }
-          sample_geometry(P.sampling_type, P.ray_radius, o, dir, row[j], far_edge(row, j, P.n_edges), pos, var);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 3; ++i) {
-            pos[i] = P.pos[3 * n + i];
-            dir[i] = P.dir[3 * n + i];
-          }
-        }
-      }
+      float pos[3], dir[3], var[3];
+      load_sample(P, n0 + tid, pos, dir, var);
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
         geo[tid * 6 + i] = pos[i];
@@ -265,7 +150,7 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
       cx.sync();
       for (int l = 0; l < P.n_sdf; ++l) {
         const Layer& L = P.lsdf[l];
-        layer_gemm(cx, P, L, smem, acc);
+        gemm(cx, P, L, smem, acc);
         const float* bl = P.w + L.b_off;
         const bool last = (l == P.n_sdf - 1);
         const int col = kSub * sub + sg;  // the sample's column in the colour trunk
@@ -275,7 +160,7 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
           for (int j = 0; j < 4; ++j) {
             const int ch = 4 * cg + 64 * i + j;
             float y, d1;
-            act_fd(P.act, acc[i][j][0] + NEUS_LDG(bl + ch), y, d1);
+            act_fd(P.act, acc[i][j][0] + LDG(bl + ch), y, d1);
             const float4 o = make_float4(y, d1 * acc[i][j][1], d1 * acc[i][j][2], d1 * acc[i][j][3]);
             if (!last) {
               *reinterpret_cast<float4*>(H + ch * kT + 4 * sg) = o;
@@ -299,7 +184,7 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
       if (n < P.n) {
         const float s = sdfv[tid];
         P.sdf[n] = s;
-        P.density[n] = sdf_density(s, NEUS_LDG(P.w + P.var_off));
+        P.density[n] = sdf_density(s, LDG(P.w + P.var_off));
         if (P.normal) {
 #pragma unroll
           for (int i = 0; i < 3; ++i) P.normal[3 * n + i] = X[(x_normal + i) * kT + tid];
@@ -310,14 +195,14 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
     // ---- colour trunk on the 64 samples (neus.py:144-149) ----
     for (int l = 0; l < P.n_col; ++l) {
       const Layer& L = P.lcol[l];
-      layer_gemm(cx, P, L, smem, acc);
+      gemm(cx, P, L, smem, acc);
       const float* bl = P.w + L.b_off;
 #pragma unroll
       for (int i = 0; i < 4; ++i)
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const int ch = 4 * cg + 64 * i + j;
-          const float b = NEUS_LDG(bl + ch);
+          const float b = LDG(bl + ch);
           float4 o;
           float d1;
           act_fd(P.act, acc[i][j][0] + b, o.x, d1);
@@ -335,8 +220,8 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
       float o[3];
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        float a = NEUS_LDG(wh + 3 * kW + c);
-        for (int k = 0; k < kW; ++k) a = fmaf(NEUS_LDG(wh + c * kW + k), H[k * kT + tid], a);
+        float a = LDG(wh + 3 * kW + c);
+        for (int k = 0; k < kW; ++k) a = fmaf(LDG(wh + c * kW + k), H[k * kT + tid], a);
         float d1;
         act_fd(P.act, a, o[c], d1);
       }
@@ -350,20 +235,12 @@ __device__ __forceinline__ void tile_program(Ctx& cx, const Params& P, float* sm
   }
 }
 
-// torch Linear weight [out][in] -> entry (k, c) of the packed [in padded][256] block
-__device__ __forceinline__ float pack_entry(const float* w, int n_in, int n_out, int k, int c) {
-  return (k < n_in && c < n_out) ? w[(size_t)c * n_in + k] : 0.f;
-}
+// entry (k, c) of a layer's packed [in padded][256] block
+__device__ __forceinline__ float pack_entry(const float* w, int n_in, int n_out, int k, int c) { return pack_fwd(w, n_in, n_out, k, c); }
 
 // ---------------------------------------------------------------------------------------------
 // host: layer table from the constructor arguments (neus.py:83-98)
 // ---------------------------------------------------------------------------------------------
-inline bool is_skip(const neddf_neus_config_t* c, int lid) {
-  for (int i = 0; i < c->n_skips; ++i)
-    if (c->skips[i] == lid) return true;
-  return false;
-}
-
 // layers_sdf.0 .. layers_sdf.{Ls-1}, layers_col.0 .. layers_col.{Lc}; returns the count
 inline int layer_shapes(const neddf_neus_config_t* c, int* sin, int* sout) {
   const int in_sdf = 6 * c->embed_pos_rank, W = c->sdf_layer_width;

@@ -1,7 +1,7 @@
 // NeuS field variant (SURVEY 8(f) item 3): the reference's NeuS network as one persistent CUDA-core kernel.
 // The tile program (index arithmetic, activations, density) lives in neus_kernel.cuh, which is also compiled by
-// g++ into a host emulation for the CPU tests; this file supplies the CUDA thread context, the weight packing
-// kernels and the C ABI (neddf_neus_*).  Forward only, fp32 FMA (parity class of the fp32 NeDDF engine).
+// g++ into a host emulation for the CPU tests; this file supplies the kernel, the weight packing and the C ABI
+// (neddf_neus_*).  Forward only, fp32 FMA (parity class of the fp32 NeDDF engine).
 #include "neus_kernel.cuh"
 
 #include <algorithm>
@@ -10,32 +10,10 @@
 namespace neddf {
 namespace neus {
 
-struct CudaCtx {
-  int tid, block, nblocks;
-  __device__ __forceinline__ void sync() { __syncthreads(); }
-  __device__ __forceinline__ void cp16(void* smem, const void* gmem) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
-  }
-  __device__ __forceinline__ void cp_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-  __device__ __forceinline__ void cp_wait_1() { asm volatile("cp.async.wait_group 1;" ::: "memory"); }
-  __device__ __forceinline__ void cp_wait_0() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-};
-
 __global__ void __launch_bounds__(kThreads, 1) neus_forward_kernel(const __grid_constant__ Params P) {
   extern __shared__ __align__(16) float smem[];
   CudaCtx cx{(int)threadIdx.x, (int)blockIdx.x, (int)gridDim.x};
   tile_program(cx, P, smem);
-}
-
-__global__ void neus_pack_kernel(const float* __restrict__ w, const float* __restrict__ b, int n_in, int n_out, int k_pad,
-                                 float* __restrict__ dst_w, float* __restrict__ dst_b) {
-  const int total = k_pad * kW;
-  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
-    const int k = idx / kW, c = idx - k * kW;
-    dst_w[idx] = pack_entry(w, n_in, n_out, k, c);
-  }
-  if (blockIdx.x == 0)
-    for (int c = threadIdx.x; c < kW; c += blockDim.x) dst_b[c] = c < n_out ? b[c] : 0.f;
 }
 
 // colour output layer [3][256] + 3 biases as stored by torch, and the variance parameter
@@ -115,7 +93,7 @@ extern "C" int32_t neddf_neus_set_weights(neddf_neus_t* h, const float* const* d
   const neus::Params& P = h->proto;
   for (int t = 0; t < n_layers - 1; ++t) {
     const neus::Layer& ly = (t < P.n_sdf) ? P.lsdf[t] : P.lcol[t - P.n_sdf];
-    neus::neus_pack_kernel<<<64, 256, 0, s>>>(d_w[t], d_b[t], h->shape_in[t], h->shape_out[t], ly.k_pad, h->d_w + ly.w_off, h->d_w + ly.b_off);
+    simt::pack_layer_kernel<<<64, 256, 0, s>>>(d_w[t], d_b[t], h->shape_in[t], h->shape_out[t], ly, h->d_w);
     NEDDF_LAUNCH_CHECK();
   }
   neus::neus_pack_head_kernel<<<1, 256, 0, s>>>(d_w[n_layers - 1], d_b[n_layers - 1], d_variance, h->d_w + P.head_off, h->d_w + P.var_off);

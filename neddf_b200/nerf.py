@@ -1,16 +1,16 @@
 """Drop-in for neddf.network.NeRF (neddf/network/nerf.py:13-178) on the B200 path: same constructor, same
 module / state_dict layout (``layers.N``, ``outL_density``, ``outL_color.0`` / ``.2``), ``forward(Sampling)`` and
-``set_iter``; the network itself runs in one CUDA kernel (``csrc/nerf_simt.cu`` behind ``neddf_nerf_*``).
+``set_iter``; the network itself runs in one CUDA kernel (``csrc/nerf.cu`` behind ``neddf_nerf_*``).
 
 Scope (SURVEY 8(f) item 3): inference - ``forward`` / ``forward_rays`` under ``torch.no_grad()``, i.e. everything
 ``NeRFRender.render_image`` and ``render_rays`` in eval need.  By default a call with autograd enabled on trainable
 parameters raises (train it with the reference, load the checkpoint here).  No CPU / PyTorch fallback.
 
 Training (opt-in: ``net.training_kernels = True`` or NEDDF_NERF_TRAIN=1): the backward of the autograd graph of
-nerf.py:107-165 with respect to the parameters runs in ``csrc/nerf_train.cu`` (forward recomputed per tile, data
-gradients in fp32 FMA) + ``neddf_wgrad`` / ``neddf_colsum_value_rows`` (weight / bias gradients).  That kernel has so far
-been validated through the host emulation of its tile program only (tests/test_nerf_train_emul.py: the real reference's
-autograd gradients, sanitizers) - it was written after the round's GPU budget was spent - hence the opt-in."""
+nerf.py:107-165 with respect to the parameters runs in the training kernel of ``csrc/nerf.cu`` (the forward's tile
+program, recomputed per tile, then the data gradients in fp32 FMA) + ``neddf_wgrad`` / ``neddf_colsum_value_rows``
+(weight / bias gradients).  That kernel has so far been validated through the host emulation of its tile program only
+(tests/test_nerf_train_emul.py: the real reference's autograd gradients, sanitizers), hence the opt-in."""
 import ctypes as C
 import math
 import os
@@ -79,7 +79,7 @@ class _NerfTrainFn(torch.autograd.Function):
         GC1 = torch.empty(n, W, device=device, dtype=torch.float32)
         GZD = torch.empty(n, device=device, dtype=torch.float32)
         lib = L.lib()
-        h = net._train_field(device)
+        h = net._kernel_handle(device, "_train")
         stream = L.stream_ptr(device)
         with torch.cuda.device(device):
             if from_rays:
@@ -172,7 +172,7 @@ class NeRF(BaseNeuralField):
         self._handle_device = None
         self._packed_key = None
         self._profile_events = None
-        # training backward (csrc/nerf_train.cu): opt-in until it has been run on hardware (module docstring)
+        # training backward (neddf_nerf_train_*): opt-in until it has been run on hardware (module docstring)
         self.training_kernels = os.environ.get("NEDDF_NERF_TRAIN", "0") not in ("", "0")
         self._train_handle = None
         self._train_handle_device = None
@@ -185,31 +185,42 @@ class NeRF(BaseNeuralField):
     def _lowpass_list(self) -> List[float]:
         return lowpass_scale(self.embed_pos_rank, self.lowpass_alpha)
 
-    def _train_field(self, device: torch.device):
-        """Handle of the training-backward kernel (forward + transposed weight packs), re-packed when a parameter changed."""
+    def _kernel_handle(self, device: torch.device, kind: str):
+        """Handle of neddf_nerf_* (kind "") or of the training backward's neddf_nerf_train_* (kind "_train", which also
+        holds the transposed weight packs) on ``device``: created on first use or a device change, re-packed when a
+        parameter changed."""
         lib = L.lib()
-        if self._train_handle is None or self._train_handle_device != device:
-            self._release_train()
+        api = "neddf_nerf" + kind
+        if getattr(self, kind + "_handle") is None or getattr(self, kind + "_handle_device") != device:
+            self._release_handle(kind)
             h = C.c_void_p()
             with torch.cuda.device(device):
                 cfg = self._config_struct()
-                L.check(lib.neddf_nerf_train_create(C.byref(cfg), C.byref(h)), "nerf_train_create")
-            self._train_handle, self._train_handle_device = h, device
+                L.check(getattr(lib, api + "_create")(C.byref(cfg), C.byref(h)), api[6:] + "_create")
+            setattr(self, kind + "_handle", h)
+            setattr(self, kind + "_handle_device", device)
         layers = self._ordered_layers()
         key = tuple((p.data_ptr(), p._version) for l in layers for p in (l.weight, l.bias))
-        if key != self._train_packed_key:
+        if key != getattr(self, kind + "_packed_key"):
+            for l in layers:
+                if l.weight.dtype != torch.float32 or not l.weight.is_contiguous() or l.weight.device != device:
+                    raise RuntimeError("neddf_b200: parameters must be contiguous fp32 tensors on the module's device")
             n = len(layers)
             ws = (C.c_void_p * n)(*[l.weight.data_ptr() for l in layers])
             bs = (C.c_void_p * n)(*[l.bias.data_ptr() for l in layers])
             with torch.cuda.device(device):
-                L.check(lib.neddf_nerf_train_set_weights(self._train_handle, ws, bs, n, L.stream_ptr(device)), "nerf_train_set_weights")
-            self._train_packed_key = key
-        return self._train_handle
+                L.check(getattr(lib, api + "_set_weights")(getattr(self, kind + "_handle"), ws, bs, n, L.stream_ptr(device)),
+                        api[6:] + "_set_weights")
+            setattr(self, kind + "_packed_key", key)
+        return getattr(self, kind + "_handle")
 
-    def _release_train(self) -> None:
-        if self._train_handle is not None:
-            L.lib().neddf_nerf_train_destroy(self._train_handle)
-        self._train_handle, self._train_handle_device, self._train_packed_key = None, None, None
+    def _release_handle(self, kind: str) -> None:
+        h = getattr(self, kind + "_handle", None)
+        if h is not None:
+            getattr(L.lib(), "neddf_nerf" + kind + "_destroy")(h)
+        setattr(self, kind + "_handle", None)
+        setattr(self, kind + "_handle_device", None)
+        setattr(self, kind + "_packed_key", None)
 
     def _config_struct(self) -> L.NerfConfig:
         c = L.NerfConfig()
@@ -225,11 +236,8 @@ class NeRF(BaseNeuralField):
         return c
 
     def _release(self) -> None:
-        if self._handle is not None:
-            L.lib().neddf_nerf_destroy(self._handle)
-        self._handle, self._handle_device, self._packed_key = None, None, None
-        if getattr(self, "_train_handle", None) is not None:
-            self._release_train()
+        self._release_handle("")
+        self._release_handle("_train")
 
     def __del__(self):
         try:
@@ -238,30 +246,10 @@ class NeRF(BaseNeuralField):
             pass
 
     def _field(self, device: torch.device):
-        lib = L.lib()
         if device.type != "cuda":
             raise RuntimeError("neddf_b200.NeRF runs on CUDA devices only: move the module with .to('cuda') "
                                "(the hot path has no CPU implementation)")
-        if self._handle is None or self._handle_device != device:
-            self._release()
-            h = C.c_void_p()
-            with torch.cuda.device(device):
-                cfg = self._config_struct()
-                L.check(lib.neddf_nerf_create(C.byref(cfg), C.byref(h)), "nerf_create")
-            self._handle, self._handle_device = h, device
-        layers = self._ordered_layers()
-        key = tuple((p.data_ptr(), p._version) for l in layers for p in (l.weight, l.bias))
-        if key != self._packed_key:
-            for l in layers:
-                if l.weight.dtype != torch.float32 or not l.weight.is_contiguous() or l.weight.device != device:
-                    raise RuntimeError("neddf_b200: parameters must be contiguous fp32 tensors on the module's device")
-            n = len(layers)
-            ws = (C.c_void_p * n)(*[l.weight.data_ptr() for l in layers])
-            bs = (C.c_void_p * n)(*[l.bias.data_ptr() for l in layers])
-            with torch.cuda.device(device):
-                L.check(lib.neddf_nerf_set_weights(self._handle, ws, bs, n, L.stream_ptr(device)), "nerf_set_weights")
-            self._packed_key = key
-        return self._handle
+        return self._kernel_handle(device, "")
 
     def _apply(self, fn, *a, **k):
         r = super()._apply(fn, *a, **k)
@@ -291,7 +279,7 @@ class NeRF(BaseNeuralField):
             raise NotImplementedError(
                 "neddf_b200.NeRF is forward-only on the B200 path by default: wrap the call in torch.no_grad() / use "
                 "render_image, or train with the reference and load the checkpoint.  The training backward kernel "
-                "(csrc/nerf_train.cu) is opt-in - net.training_kernels = True or NEDDF_NERF_TRAIN=1 - until it has been "
+                "(neddf_nerf_train_*) is opt-in - net.training_kernels = True or NEDDF_NERF_TRAIN=1 - until it has been "
                 "run on hardware (so far: host emulation against the reference's autograd gradients)")
         return True
 

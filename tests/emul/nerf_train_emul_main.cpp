@@ -1,6 +1,6 @@
-// Sanitizer driver for the emulated NeRF training-backward kernel (TEST INFRASTRUCTURE): see neus_emul_main.cpp.
-// Exact-size buffers (a store past sample n - 1 is a heap overflow), full + ragged tiles, two CTAs, explicit samples
-// and fused ray geometry.  Exit code 0 = clean.
+// Sanitizer driver for the emulated NeRF kernels, forward and training backward (TEST INFRASTRUCTURE): see
+// neus_emul_main.cpp.  Exact-size buffers (a store past sample n - 1 is a heap overflow), full + ragged tiles, two CTAs,
+// explicit samples and fused ray geometry.  Exit code 0 = clean.
 #include "nerf_train_emul.cpp"
 
 #include <stdio.h>
@@ -55,7 +55,14 @@ static int run(const neddf_nerf_config_t& cfg, int n, bool rays, unsigned seed) 
   for (float v : GC1) sum += v;
   for (float v : GZD) sum += v;
   printf("rc %d checksum %.6f (%lld samples)\n", rc, sum, total);
-  return (rc == 0 && sum == sum) ? 0 : 1;
+  std::vector<float> den(total), col(3 * total);
+  const int rc_f = nerf_forward_emul(&cfg, wp.data(), bp.data(), nl, lowpass, rays ? nullptr : pos.data(), rays ? nullptr : dir.data(),
+                                     rays ? nullptr : var.data(), rays ? rd.data() : nullptr, rays ? ro.data() : nullptr,
+                                     rays ? dists.data() : nullptr, n, n_edges, NEDDF_SAMPLING_CONE, 2.6e-4f, den.data(), col.data(), 2);
+  double sum_f = 0;
+  for (long long i = 0; i < total; ++i) sum_f += den[i] + col[3 * i] + col[3 * i + 2];
+  printf("forward rc %d checksum %.6f (%lld samples)\n", rc_f, sum_f, total);
+  return (rc == 0 && sum == sum && rc_f == 0 && sum_f == sum_f) ? 0 : 1;
 }
 
 int main() {

@@ -1,6 +1,6 @@
 """(child process of tests/test_zzz_nerf_train_gpu.py - run as `python -m tests.nerf_train_gpu_child <check> <case>`)
 
-NeRF variant, training backward on the GPU (csrc/nerf_train.cu + neddf_wgrad behind neddf_b200.NeRF with
+NeRF variant, training backward on the GPU (the training kernel of csrc/nerf.cu + neddf_wgrad behind neddf_b200.NeRF with
 training_kernels=True) against the REAL reference's autograd gradients (tests/golden/make_nerf_train_golden.py).
 
 STATUS - read before trusting a green or red mark here: this kernel was written after the round's GPU budget was

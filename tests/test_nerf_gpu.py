@@ -1,4 +1,4 @@
-"""NeRF field variant on the GPU (csrc/nerf_simt.cu behind neddf_b200.NeRF) against goldens recorded from the REAL
+"""NeRF field variant on the GPU (csrc/nerf.cu behind neddf_b200.NeRF) against goldens recorded from the REAL
 reference (tests/golden/make_nerf_golden.py) and the oracle restatement: per-sample field outputs with explicit
 samples and with the fused ray geometry, render_rays through NeRFRender with the recorded uniforms, the image path."""
 import numpy as np

@@ -1,12 +1,13 @@
-"""The NeRF variant's training-backward kernel (csrc/nerf_train.cu), executed on the CPU.
+"""The NeRF variant's kernels (csrc/nerf.cu), forward and training backward, executed on the CPU.
 
-Its tile program (neddf_b200/csrc/nerf_train_kernel.cuh) is compiled by g++ into tests/emul/libnerf_train_emul.so (a CTA =
-256 OS threads, pthread barrier for __syncthreads) and run on the samples and the upstream gradients (d loss / d density,
+Their tile program (neddf_b200/csrc/nerf_train_kernel.cuh) is compiled by g++ into tests/emul/libnerf_train_emul.so
+(a CTA = 256 OS threads, pthread barrier for __syncthreads).  The forward is checked against the field goldens of the real reference and
+the oracle.  The backward is run on the samples and the upstream gradients (d loss / d density,
 d loss / d colour per sample, captured with tensor hooks) of fixtures recorded from the REAL reference's autograd
 (tests/golden/make_nerf_train_golden.py).  The parameter gradients are then assembled exactly as the GPU path does -
 gW = X^T G over all samples, bias = column sums - with numpy standing in for neddf_wgrad, and compared with the
-reference's.  STATUS of the kernel itself: not yet run on hardware (the round's GPU budget was spent when it was
-written); tests/test_nerf_train_gpu.py holds the GPU tests."""
+reference's.  STATUS of the backward kernel itself: not yet passed on hardware; tests/test_zzz_nerf_train_gpu.py holds
+its GPU tests."""
 import ctypes as C
 import json
 import os
@@ -18,7 +19,8 @@ import pytest
 import torch
 
 from oracle import neddf_oracle as orc
-from tests.helpers import GOLDEN, assert_parity, nerr
+from tests.helpers import GOLDEN, PARITY_TOL, assert_parity, nerr
+from tests.test_nerf_oracle import NerfCase
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "emul", "nerf_train_emul.cpp")
@@ -56,12 +58,14 @@ def emul():
     if shutil.which("g++") is None or not os.path.isdir(CUDA_INC):
         pytest.skip("g++ / CUDA headers not available")
     deps = [SRC, os.path.join(HERE, "emul", "emul_common.h"), os.path.join(HERE, "..", "neddf_b200", "csrc", "nerf_train_kernel.cuh"),
-            os.path.join(HERE, "..", "neddf_b200", "csrc", "common.cuh"), os.path.join(HERE, "..", "include", "neddf_b200.h")]
+            os.path.join(HERE, "..", "neddf_b200", "csrc", "simt_mlp.cuh"), os.path.join(HERE, "..", "neddf_b200", "csrc", "common.cuh"),
+            os.path.join(HERE, "..", "include", "neddf_b200.h")]
     if not os.path.exists(LIB) or any(os.path.getmtime(d) > os.path.getmtime(LIB) for d in deps):
         subprocess.run(["g++", "-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", "-I" + CUDA_INC, SRC, "-o", LIB],
                        check=True)
     lib = C.CDLL(LIB)
     lib.nerf_train_emul.restype = C.c_int
+    lib.nerf_forward_emul.restype = C.c_int
     return lib
 
 
@@ -103,6 +107,80 @@ def run_backward(lib, nc, alpha, ws, bs, ray_dir, ray_orig, dists, sampling_type
     assert rc == 0
     assert all(np.isfinite(v).all() for v in buf.values())
     return buf, gd, gc
+
+
+def run_forward(lib, nc, alpha, ws, bs, sampling_type, pos=None, dirs=None, var=None, rays=None, nblocks=2):
+    """The emulated forward kernel on explicit samples (pos, dirs, var [..., 3]) or rays ((ray_dir, ray_orig, dists),
+    fused geometry): {'density': [...], 'color': [..., 3]}."""
+    def p(a):
+        return None if a is None else a.ctypes.data_as(FP)
+
+    if rays is not None:
+        rd, ro, di = (np.ascontiguousarray(t.numpy(), np.float32) for t in rays)
+        n, n_edges = di.shape
+        shape = di.shape
+        pa = da = va = None
+    else:
+        pa, da, va = (np.ascontiguousarray(t.reshape(-1, 3).numpy(), np.float32) for t in (pos, dirs, var))
+        rd = ro = di = None
+        n, n_edges, shape = pa.shape[0], 0, tuple(pos.shape[:-1])
+    total = int(np.prod(shape))
+    density, color = np.full((total,), np.nan, np.float32), np.full((total, 3), np.nan, np.float32)
+    lowpass = orc.lowpass_scale(nc.embed_pos_rank, alpha).numpy().astype(np.float32)
+    wp = (FP * len(ws))(*[p(a) for a in ws])
+    bp = (FP * len(bs))(*[p(a) for a in bs])
+    cfg = cfg_struct(nc)
+    radius = orc.CONE_RAY_RADIUS if sampling_type == "cone" else 0.0
+    rc = lib.nerf_forward_emul(C.byref(cfg), wp, bp, len(ws), p(lowpass), p(pa), p(da), p(va), p(rd), p(ro), p(di), C.c_longlong(n),
+                               C.c_int(n_edges), C.c_int({"point": 0, "cone": 1}[sampling_type]), C.c_float(radius), p(density),
+                               p(color), C.c_int(nblocks))
+    assert rc == 0
+    return {"density": density.reshape(shape), "color": color.reshape(shape + (3,))}
+
+
+def _case_weights(c: NerfCase, tag: str):
+    """torch layout ([out,in] weights, [out] biases) of a NerfCase in the order of neddf_nerf_layer_shapes."""
+    pre = f"w_{tag}." if f"w_{tag}.layers.0.weight" in c.z else "w_fine."
+    names = [n for n, _, _ in orc.nerf_layer_shapes(c.nc)]
+    return ([np.ascontiguousarray(c.z[pre + n + ".weight"], np.float32) for n in names],
+            [np.ascontiguousarray(c.z[pre + n + ".bias"], np.float32) for n in names])
+
+
+@pytest.mark.parametrize("name", ["relu", "tanhexp"])
+def test_emulated_forward_matches_reference_goldens(emul, name):
+    """The forward kernel's coarse and fine fields, explicit samples and fused geometry, against the real reference's
+    (a slice of the rays: full + ragged tiles over two CTAs at a few seconds of emulation)."""
+    c = NerfCase(name)
+    d, o = orc.make_rays(c.t("uv"), c.cam)
+    for tag, dists, n_rays in (("coarse", orc.coarse_dists(c.rc, c.t("u_coarse")), 3), ("fine", c.t("dists_fine"), 2)):
+        sl = slice(0, n_rays)
+        ws, bs = _case_weights(c, tag)
+        pos, dd, var = orc.make_samples(c.rc, d[sl], o[sl], dists[sl])
+        fused = run_forward(emul, c.nc, c.alpha, ws, bs, c.rc.sampling_type, rays=(d[sl], o[sl], dists[sl]))
+        explicit = run_forward(emul, c.nc, c.alpha, ws, bs, c.rc.sampling_type, pos=pos, dirs=dd.contiguous(), var=var, nblocks=1)
+        for k in ("density", "color"):
+            ref = c.z[f"field_{tag}_{k}"][sl]
+            for what, got in (("explicit samples", explicit[k]), ("fused geometry", fused[k])):
+                assert got.shape == ref.shape, (tag, k, what)
+                assert np.isfinite(got).all(), (tag, k, what)
+                assert nerr(got, ref) < PARITY_TOL, (tag, k, what, nerr(got, ref))
+
+
+def test_emulated_forward_ragged_tiles(emul):
+    """Sample counts that are not multiples of the 64-sample tile, against the oracle field on the same samples."""
+    c = NerfCase("relu")
+    ws, bs = _case_weights(c, "fine")
+    g = torch.Generator().manual_seed(5)
+    for n in (1, 63, 65, 1000):
+        pos = (torch.rand(1, n, 3, generator=g) * 2 - 1)
+        dd = torch.nn.functional.normalize(torch.randn(1, n, 3, generator=g), dim=-1)
+        var = torch.rand(1, n, 3, generator=g) * 1e-3
+        out = run_forward(emul, c.nc, c.alpha, ws, bs, "cone", pos=pos, dirs=dd, var=var)
+        with torch.no_grad():
+            ref = orc.nerf_forward(c.params("fine"), c.nc, c.alpha, pos, dd, var)
+        for k in ("density", "color"):
+            a, r = out[k], ref[k].numpy()
+            assert np.abs(a - r).max() <= PARITY_TOL * max(np.abs(r).max(), 1.0), (n, k)
 
 
 def oracle_grads(c: TrainCase, dtype):
@@ -369,12 +447,12 @@ def _san_build(tmp_path, name, flags):
 
 def test_emulated_backward_under_sanitizers(emul, tmp_path):
     """AddressSanitizer + UBSan (memcheck: exact-size buffers, float4 alignment) and ThreadSanitizer (racecheck, best
-    effort) on the emulated training-backward kernel (the negative controls that show the detectors see this kind of code
+    effort) on the emulated forward and training-backward kernels (the negative controls that show the detectors see this kind of code
     live in tests/test_neus_emul.py: same harness, same GEMM loop)."""
     env = dict(os.environ, TSAN_OPTIONS="halt_on_error=0 exitcode=66", ASAN_OPTIONS="detect_leaks=0")
     r = subprocess.run([_san_build(tmp_path, "asan", ["-fsanitize=address,undefined", "-fno-sanitize-recover=all"])], capture_output=True,
                        text=True, env=env, timeout=600)
     assert r.returncode == 0 and "runtime error" not in r.stderr and "AddressSanitizer" not in r.stderr, r.stderr[-1500:]
-    assert r.stdout.count("rc 0 checksum") == 2
+    assert r.stdout.count("rc 0 checksum") == 4  # two configurations, forward and backward
     r = subprocess.run([_san_build(tmp_path, "tsan", ["-fsanitize=thread"])], capture_output=True, text=True, env=env, timeout=600)
     assert r.returncode == 0 and "ThreadSanitizer" not in r.stderr, r.stderr[-1500:]

@@ -29,7 +29,8 @@ def emul():
     if shutil.which("g++") is None or not os.path.isdir(CUDA_INC):
         pytest.skip("g++ / CUDA headers not available")
     deps = [SRC, os.path.join(HERE, "emul", "emul_common.h"), os.path.join(HERE, "..", "neddf_b200", "csrc", "neus_kernel.cuh"),
-            os.path.join(HERE, "..", "neddf_b200", "csrc", "common.cuh"), os.path.join(HERE, "..", "include", "neddf_b200.h")]
+            os.path.join(HERE, "..", "neddf_b200", "csrc", "simt_mlp.cuh"), os.path.join(HERE, "..", "neddf_b200", "csrc", "common.cuh"),
+            os.path.join(HERE, "..", "include", "neddf_b200.h")]
     if not os.path.exists(LIB) or any(os.path.getmtime(d) > os.path.getmtime(LIB) for d in deps):
         subprocess.run(["g++", "-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", "-I" + CUDA_INC,
                         SRC, "-o", LIB], check=True)

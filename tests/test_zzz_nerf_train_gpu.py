@@ -1,4 +1,4 @@
-"""NeRF variant, training backward on the GPU: first hardware run of csrc/nerf_train.cu (see tests/nerf_train_gpu_child.py
+"""NeRF variant, training backward on the GPU: first hardware run of the training kernel of csrc/nerf.cu (see tests/nerf_train_gpu_child.py
 for the checks and their status).  Each check runs in a CHILD PROCESS with a timeout and this file is collected last:
 a fault or a hang of a kernel that has never run on hardware cannot poison the CUDA context of the validated suite.
 NON-STRICT expected failures: XPASS = the first hardware run succeeded, XFAIL = a finding for the next round."""
@@ -9,7 +9,7 @@ import sys
 import pytest
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.xfail(strict=False, reason="first hardware run of csrc/nerf_train.cu (validated by host emulation only)")]
+              pytest.mark.xfail(strict=False, reason="first hardware run of the NeRF training kernel (validated by host emulation only)")]
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 

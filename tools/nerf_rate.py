@@ -1,4 +1,4 @@
-"""Throughput of the NeRF variant's kernel (csrc/nerf_simt.cu): fused-ray forward on a slice of the bench frame.
+"""Throughput of the NeRF variant's kernel (csrc/nerf.cu): fused-ray forward on a slice of the bench frame.
 FLOP per evaluation = 2 x sum of in x out over its linear layers (padding not counted)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -1,4 +1,4 @@
-"""NeRF variant, training step probe (csrc/nerf_train.cu + neddf_wgrad; opt-in path, DESIGN 4.7): forward + backward of
+"""NeRF variant, training step probe (the training kernel of csrc/nerf.cu + neddf_wgrad; opt-in path, DESIGN 4.7): forward + backward of
 NeRF.forward_rays on a slice of the bench frame, and the worst parameter-gradient distance from torch autograd through the
 oracle on a small batch.  First thing to run when a GPU is available again (the kernel has only run in host emulation)."""
 import os, sys
